@@ -50,7 +50,16 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--sweep", action="store_true", default=True, help="(N>1) also report allreduce bus GB/s at the model's bucket sizes and 256 MiB")
     ap.add_argument("--no-sweep", dest="sweep", action="store_false")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed on rank 0 as DIR/<name>.npy (float32): loss, logits, "
+                         "the averaged gradients and the updated parameters; arrays over %d elements as the same seeded sample "
+                         "of positions in every run, so two builds can be compared output for output.  Such a run uses deterministic "
+                         "cuDNN / cuBLAS algorithms instead of autotuned ones, so its timing is not the headline number; two such runs "
+                         "of one build on the same GPU model and library versions give the same bits, other GPUs or libraries need not" % (1 << 21))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1: the timed region is --steps optimizer steps")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -198,7 +207,15 @@ class Trainer:
         self.args, self.rank, self.world = args, rank, world
         self.device = torch.device("cuda", local_rank)
         torch.cuda.set_device(self.device)
-        torch.backends.cudnn.benchmark = True
+        torch.backends.cudnn.benchmark = not args.dump_outputs
+        if args.dump_outputs:
+            # the autotuner picks algorithms by timing, and SGD at lr 0.1 grows the last-bit differences between two picks into
+            # different weights within the timed steps (ResNet-50, --steps 20 --warmup 5 on a B200 at 1000 W: two autotuned runs
+            # ended at loss 5.56 and 3.72): fixed deterministic algorithms make two runs, and two builds, comparable.  Not
+            # warn_only: with it cuDNN attention's backward stays non-deterministic (GPT-2 dumps differed), and an op that has
+            # no deterministic implementation must stop the run rather than break the promise silently
+            torch.backends.cudnn.deterministic = True
+            torch.use_deterministic_algorithms(True)
         self.comm = None
         self.is_image = args.model == "resnet50"
         model = build_model(args.model, self.device)
@@ -262,17 +279,47 @@ class Trainer:
         return float(t.max().item())
 
     # -- one optimizer step -----------------------------------------------------------------------------------
-    def step(self, x, y):
+    def step(self, x, y, keep=False):
+        """keep: hold on to this step's loss and logits for dump_outputs (only asked of the last timed step)."""
         torch = self.torch
         with torch.autocast("cuda", dtype=torch.bfloat16):
             if self.is_image:
-                loss = self.loss_fn(self.ddp(x), y)
+                logits = self.ddp(x)
+                loss = self.loss_fn(logits, y)
             else:
-                loss = self.ddp(input_ids=x, labels=y).loss
+                out = self.ddp(input_ids=x, labels=y)
+                loss, logits = out.loss, out.logits
+                del out
+        if keep:
+            self.last_loss, self.last_logits = loss.detach(), logits.detach()
+        del logits
         self.opt.zero_grad(set_to_none=True)
         loss.backward()
         self.opt.step()
         return loss
+
+    def dump_outputs(self, out_dir, max_elems=1 << 21):
+        """What the last timed step handed its caller: loss, logits, the averaged gradients (param.grad, in parameter
+        order) and the parameters after the optimizer step, as float32 .npy files.  An array larger than max_elems is
+        written as the elements at a sorted sample of positions drawn with a fixed seed from its size, so the same
+        positions are taken in every run."""
+        import numpy as np
+
+        torch = self.torch
+        params = [p for p in self.ddp.parameters() if p.requires_grad]
+        arrays = {
+            "loss": self.last_loss.float().reshape(1),
+            "logits": self.last_logits.float().reshape(-1),
+            "grads": torch.cat([p.grad.detach().float().reshape(-1) for p in params]),
+            "params": torch.cat([p.detach().float().reshape(-1) for p in params]),
+        }
+        os.makedirs(out_dir, exist_ok=True)
+        for name, t in arrays.items():
+            n = t.numel()
+            if n > max_elems:
+                idx = np.sort(np.random.default_rng(n).choice(n, size=max_elems, replace=False))
+                t = t[torch.from_numpy(idx).to(t.device)]
+            np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
 
     def run_resident(self, steps, warmup):
         """`value`: batch already in HBM."""
@@ -297,9 +344,10 @@ class Trainer:
         profiled = bool(os.environ.get("BENCH_CUDA_PROFILER"))  # ncu --profile-from-start off: capture the timed region only
         if profiled:
             torch.cuda.profiler.start()
+        keep = bool(self.args.dump_outputs)
         e0.record()
-        for _ in range(steps):
-            loss = self.step(x, y)
+        for i in range(steps):
+            loss = self.step(x, y, keep=keep and i == steps - 1)
         e1.record()
         self.barrier()
         if profiled:
@@ -569,6 +617,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", str(rank)))
     if world != args.gpus and rank == 0:
         print(f"[bench] note: --gpus {args.gpus} but WORLD_SIZE={world}; using WORLD_SIZE", file=sys.stderr)
+    if args.dump_outputs:
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")  # reproducible cuBLAS; read when its first handle is made
     import torch
 
     if not torch.cuda.is_available():
@@ -581,6 +631,8 @@ def main():
     tr = Trainer(args, rank, world, local_rank)
     elapsed, last_loss, clocks, launches, kernel, nv0, nv1 = tr.run_resident(args.steps, args.warmup)
     elapsed = tr.max_over_ranks(elapsed)
+    if args.dump_outputs and rank == 0:  # before run_e2e trains on
+        tr.dump_outputs(args.dump_outputs)
     samples = args.batch * world * args.steps
     n_grad = int(sum(p.numel() for p in tr.ddp.parameters() if p.requires_grad))
     line = {
@@ -609,6 +661,8 @@ def main():
         "gpu_launches": launches,
         "last_loss": round(last_loss, 4),
     }
+    if args.dump_outputs:
+        line["deterministic_algorithms"] = "outputs dumped: cuDNN autotuning off, so this is not the headline timing"
     if args.impl == "reference_tuned":
         line["tuned"] = "gradient_as_bucket_view=True, static_graph=True (attribution arm; the headline reference arm uses DDP's defaults)"
     if not args.no_e2e:

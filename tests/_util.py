@@ -1,6 +1,9 @@
 """Shared helpers for the parity tests (CPU side: numpy + oracle; GPU side: torch tensors)."""
 from __future__ import annotations
 
+import dataclasses
+import enum
+
 import numpy as np
 
 import oracle
@@ -36,6 +39,27 @@ def make_inputs(world: int, n: int, seed: int, kind: str = "randn") -> list:
             raise ValueError(kind)
         out.append(x)
     return out
+
+
+def encode(v, subst: dict):
+    """JSON form of a value crossing the Runner -> scheduler boundary (tests/golden/reference_dropin.json): dataclasses
+    and enums by class name, other objects by type name only, and every ``subst`` key inside a string replaced by its
+    token, so that run-specific paths and ids compare equal."""
+    if isinstance(v, enum.Enum):
+        return {"__enum__": [type(v).__name__, v.name]}
+    if dataclasses.is_dataclass(v) and not isinstance(v, type):
+        return {"__dataclass__": type(v).__name__, "fields": {f.name: encode(getattr(v, f.name), subst) for f in dataclasses.fields(v)}}
+    if isinstance(v, dict):
+        return {str(k): encode(x, subst) for k, x in v.items()}
+    if isinstance(v, (list, tuple)):
+        return [encode(x, subst) for x in v]
+    if isinstance(v, str):
+        for k, tok in subst.items():
+            v = v.replace(k, tok)
+        return v
+    if v is None or isinstance(v, (bool, int, float)):
+        return v
+    return {"__object__": type(v).__name__}
 
 
 def assert_bits_equal(got: np.ndarray, want: np.ndarray, what: str = "") -> None:

@@ -7,6 +7,8 @@
                    gradients and the three averaged results, so the oracle can be pinned against them.
   bucket_layouts.json   torch's own dist._compute_bucket_assignment_by_size over ResNet-50 / GPT-2-small /
                    BERT-base parameters (reverse order, limits [1 MiB, 25 MiB]) - layout parity fixture.
+  reference_dropin.json   every call the reference's own Runner makes on the local_cuda scheduler (factory handed to
+                   the Runner, and found as a torchx_plugins namespace plugin), with arguments and results.
 
 Run from the repo root:  python tests/golden/make_golden.py      (needs /root/reference; not needed at test time)
 """
@@ -215,8 +217,52 @@ def launcher_goldens() -> None:
     print("wrote launcher.json")
 
 
+DROPIN_PLUGIN = textwrap.dedent('''
+    from torchx.plugins import register
+
+
+    @register.scheduler(name="local_cuda")
+    def local_cuda(session_name: str, **kwargs):
+        from torchx_b200.schedulers.local_cuda_scheduler import create_scheduler
+        return create_scheduler(session_name, **kwargs)
+
+
+    @register.scheduler(name="local_cwd")
+    def local_cwd(session_name: str, **kwargs):
+        from torchx.schedulers.local_scheduler import create_scheduler
+        return create_scheduler(session_name, **kwargs)
+''')
+
+
+def dropin_traces() -> None:
+    """The reference's own Runner submits its own dist.ddp AppDef (-j 1x2, CPU/gloo toy job) to local_cuda, once with the
+    factory handed to the Runner and once through the torchx_plugins namespace plugin of INTEGRATION.md; every call the
+    Runner makes on the scheduler is recorded (tests/workers/reference_runner_driver.py)."""
+    root = os.path.dirname(os.path.dirname(HERE))
+    out = {}
+    for mode in ("factory", "plugin"):
+        with tempfile.TemporaryDirectory() as td:
+            extra = []
+            if mode == "plugin":
+                pkg = os.path.join(td, "plug", "torchx_plugins", "schedulers")
+                os.makedirs(pkg)
+                with open(os.path.join(pkg, "b200.py"), "w") as f:  # namespace packages: no __init__.py on purpose
+                    f.write(DROPIN_PLUGIN)
+                extra = [os.path.join(td, "plug")]
+            env = dict(os.environ, PYTHONPATH=os.pathsep.join([REF, *extra, root]), TORCHX_HOME=os.path.join(td, "home"))
+            trace = os.path.join(td, "trace.json")
+            cmd = [sys.executable, os.path.join(root, "tests", "workers", "reference_runner_driver.py"), mode,
+                   os.path.join(root, "examples", "toy_ddp.py"), os.path.join(td, "logs"), trace]
+            subprocess.run(cmd, check=True, cwd=td, env=env, timeout=600)
+            with open(trace) as f:
+                out[mode] = json.load(f)
+    with open(os.path.join(HERE, "reference_dropin.json"), "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+    print("wrote reference_dropin.json")
+
+
 if __name__ == "__main__":
-    what = sys.argv[1:] or ["ddp", "buckets", "launcher"]
+    what = sys.argv[1:] or ["ddp", "buckets", "launcher", "dropin"]
     if "ddp" in what:
         for w in (2, 4):
             run_reference_ddp(w)
@@ -224,3 +270,5 @@ if __name__ == "__main__":
         bucket_layouts()
     if "launcher" in what:
         launcher_goldens()
+    if "dropin" in what:
+        dropin_traces()
