@@ -186,6 +186,7 @@ int b2_allreduce(b2_comm_t* comm, void* buf, size_t n_elems, int mode, float sca
  * [begin, end) and reads them from the DEVICE pointer `src` (this rank's tensor of the bucket's dtype, dense in the
  * bucket's element order; it may alias `out`).  The table is copied into the kernel parameters by this call: it need not
  * outlive it.  `out` is this rank's bucket.  More parameters than B2_MAX_SEGMENTS: B2_EINVAL (copy in, then b2_allreduce).
+ * A NULL table, an empty segment, a NULL `src`, a gap or a table that does not cover exactly n_elems: B2_EINVAL.
  */
 #define B2_MAX_SEGMENTS 128
 typedef struct b2_segment {

@@ -8,6 +8,10 @@ import numpy as np
 
 import oracle
 
+MODES = {"f32_wire_bf16": oracle.B2O_F32_WIRE_BF16, "f32": oracle.B2O_F32, "bf16": oracle.B2O_BF16}
+WIRE = {"f32_wire_bf16": "bf16", "f32": "f32", "bf16": "bf16"}
+GUARD = 64  # canary elements on each side of every tensor a kernel writes
+
 SPECIALS = np.array(
     [0.0, -0.0, np.inf, -np.inf, np.nan, 1e-40, -1e-40, 1.17549435e-38, 3.3895314e38, -3.3895314e38, 1.0, -1.0,
      1.00390625, 1.0078125, 1.01171875, 65504.0, 1e-3, -1e-3, 255.0, 256.0, 257.0],
@@ -109,3 +113,107 @@ def assert_nvls_result(got: np.ndarray, inputs: list, scale: float, mode: int, w
             f"got {gf[bad[:8]]} exact {exact[bad[:8]]} rank-order {wf[bad[:8]]}")
         del absmax
     return {"n": int(got.size), "differ_from_rank_order": int(diff.size)}
+
+
+# ---- GPU side ------------------------------------------------------------------------------------------------------
+def devices(world: int, cuda_count: int, spread: bool) -> list:
+    """Device of each rank: one rank per GPU (skips the test without enough GPUs) or every rank on cuda:0."""
+    import pytest
+
+    if spread:
+        if cuda_count < world:
+            pytest.skip(f"needs {world} GPUs")
+        return list(range(world))
+    return [0] * world
+
+
+class World:
+    """An in-process topology (b2_comm_create_local): rank r launches on its own stream of devices[r]."""
+
+    def __init__(self, devices, stage_mb=8, timeout_s=10.0):
+        import torch
+        from torchx_b200.ddp import Communicator
+
+        self.comms = Communicator.create_local(devices, stage_mb=stage_mb)
+        self.streams = [torch.cuda.Stream(device=d) for d in devices]
+        same_device = len(set(devices)) == 1
+        for c in self.comms:
+            c.set_timeout(timeout_s)
+            if same_device:  # all kernels must be co-resident on one GPU: W ranks x grid <= #SMs (1 CTA per SM)
+                c.set_max_ctas(max(1, 128 // len(devices)))
+
+    def run(self, fn):
+        """fn(rank, comm, stream) launches that rank's work; then wait for all and check health.  fn must not allocate
+        or synchronise: the ranks launched before it spin until every peer has launched."""
+        for r, (c, s) in enumerate(zip(self.comms, self.streams)):
+            fn(r, c, s)
+        for s in self.streams:
+            s.synchronize()
+        for c in self.comms:
+            c.check()
+
+    def close(self):
+        for c in self.comms:
+            c.close()
+
+
+def host_elems(x: np.ndarray, mode: str) -> np.ndarray:
+    """fp32 values as the tensor of `mode` holds them: fp32, or bf16 bit patterns (uint16) in bf16 mode."""
+    return oracle.f32_to_bf16_bits(x) if mode == "bf16" else x
+
+
+def _int_view(a: np.ndarray) -> np.ndarray:
+    return a.view(np.uint16) if a.dtype.itemsize == 2 else a.view(np.uint32)
+
+
+def upload(h: np.ndarray, device):
+    """Host elements (fp32, or uint16 bf16 bits) -> the same bits in a float32 / bfloat16 tensor, NaN payloads included."""
+    import torch
+
+    bits = _int_view(np.ascontiguousarray(h))
+    if bits.dtype == np.uint16:
+        return torch.from_numpy(bits.view(np.int16).copy()).to(f"cuda:{device}").view(torch.bfloat16)
+    return torch.from_numpy(bits.view(np.int32).copy()).to(f"cuda:{device}").view(torch.float32)
+
+
+def to_dev(x: np.ndarray, mode: str, device):
+    h = host_elems(x, mode)
+    return upload(h, device), h
+
+
+def to_host(t, mode: str) -> np.ndarray:
+    import torch
+
+    if mode == "bf16":
+        return t.view(torch.int16).cpu().numpy().view(np.uint16)
+    return t.cpu().numpy()
+
+
+def garbage(n: int, mode: str, seed: int) -> np.ndarray:
+    """Random bit patterns (NaNs and infinities included) in the element type of `mode`."""
+    rng = np.random.default_rng(seed)
+    if mode == "bf16":
+        return rng.integers(0, 1 << 16, size=n, dtype=np.uint16)
+    return rng.integers(0, 1 << 32, size=n, dtype=np.uint32).view(np.float32)
+
+
+class Guarded:
+    """A device tensor `t` holding the host elements `h`, placed `offset` elements after GUARD canary elements and
+    followed by GUARD more, all in one allocation.  A store past either end of `t` lands in a canary, where the caching
+    allocator's slack would have hidden it."""
+
+    def __init__(self, h: np.ndarray, mode: str, device, offset: int = 0, seed: int = 0):
+        n = h.size
+        self.mode = mode
+        self.lo, self.hi = GUARD + offset, GUARD + offset + n
+        self.init = garbage(self.hi + GUARD, mode, seed)
+        _int_view(self.init)[self.lo:self.hi] = _int_view(np.ascontiguousarray(h))
+        self.full = upload(self.init, device)
+        self.t = self.full[self.lo:self.hi]
+
+    def check(self, what: str = "") -> None:
+        got = _int_view(to_host(self.full, self.mode))
+        want = _int_view(self.init)
+        for name, sl in (("before", slice(0, self.lo)), ("after", slice(self.hi, None))):
+            bad = np.flatnonzero(got[sl] != want[sl])
+            assert bad.size == 0, f"{what}: {bad.size} canary elements {name} the tensor were overwritten, first at {bad[:8]}"

@@ -68,5 +68,38 @@ def test_argument_validation_without_a_gpu():
     assert L.b2_allreduce_gather(None, ctypes.c_void_p(4096), 20, segs, 2, 0, 1.0, 0, None) == N.B2_EINVAL
     assert b"does not continue" in L.b2_last_error()
     assert L.b2_allreduce_gather(None, ctypes.c_void_p(4096), 20, segs, N.B2_MAX_SEGMENTS + 1, 0, 1.0, 0, None) == N.B2_EINVAL
+    assert b"need 1..128 segments (got 129)" in L.b2_last_error()
     assert L.b2_comm_caps(None) == N.B2_EINVAL and L.b2_comm_last_algo(None) == N.B2_EINVAL
     assert L.b2_comm_set_param(None, b"max_ctas", 1) == N.B2_EINVAL
+
+
+def _gather_table_error(table, n_elems, n_segments=None):
+    """Return code and b2_last_error() of a gather call with this (src, begin, end) table; a null communicator, so the
+    call can only get as far as the host-side validation of the table."""
+    L = N.lib()
+    segs = (N.B2Segment * max(1, len(table)))()
+    for i, (src, begin, end) in enumerate(table):
+        segs[i].src, segs[i].begin, segs[i].end = src, begin, end
+    n = len(table) if n_segments is None else n_segments
+    rc = L.b2_allreduce_gather(None, ctypes.c_void_p(4096), n_elems, segs, n, 0, 1.0, 0, None)
+    return rc, L.b2_last_error().decode()
+
+
+def test_gather_segment_table_validation_without_a_gpu():
+    ok = [(4096, 0, 10), (8192, 10, 20)]
+    assert _gather_table_error(ok, 20) == (N.B2_EINVAL, "null communicator")  # the table itself passes
+    cases = [
+        ([(4096, 0, 10), (8192, 10, 10), (8192, 10, 20)], 20, "segment 1 is empty"),
+        ([(4096, 0, 0), (8192, 0, 20)], 20, "segment 0 is empty"),
+        ([(4096, 0, 10), (None, 10, 20)], 20, "segment 1 has a null src"),
+        ([(4096, 0, 10), (8192, 10, 20)], 21, "segments cover 20 elements, bucket has 21"),
+        ([(4096, 0, 10), (8192, 10, 20)], 19, "segments cover 20 elements, bucket has 19"),
+        ([(4096, 0, 10), (8192, 9, 20)], 20, "segment 1 does not continue the bucket at element 10"),
+        ([(4096, 1, 10)], 9, "segment 0 does not continue the bucket at element 0"),
+    ]
+    for table, n_elems, msg in cases:
+        assert _gather_table_error(table, n_elems) == (N.B2_EINVAL, f"b2_allreduce_gather: {msg}"), (table, n_elems)
+    assert _gather_table_error(ok, 20, n_segments=0) == (N.B2_EINVAL, "b2_allreduce_gather: need 1..128 segments (got 0)")
+    L = N.lib()
+    assert L.b2_allreduce_gather(None, ctypes.c_void_p(4096), 20, None, 2, 0, 1.0, 0, None) == N.B2_EINVAL  # NULL table
+    assert L.b2_last_error() == b"b2_allreduce_gather: null segment table"

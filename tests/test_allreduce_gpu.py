@@ -7,83 +7,44 @@ import pytest
 import torch
 
 import oracle
-from tests._util import assert_bits_equal, assert_nvls_result, make_inputs
+from tests._util import (MODES, WIRE, Guarded, World, assert_bits_equal, assert_nvls_result, devices, host_elems, make_inputs,
+                         to_dev, to_host)
 
 pytestmark = pytest.mark.gpu
 
-MODES = {"f32_wire_bf16": oracle.B2O_F32_WIRE_BF16, "f32": oracle.B2O_F32, "bf16": oracle.B2O_BF16}
-WIRE = {"f32_wire_bf16": "bf16", "f32": "f32", "bf16": "bf16"}
 SIZES = [1, 7, 8, 9, 1023, 1024, 1025, 4099, 32771, (1 << 18) + 5]
 
 
-def _devices(world, cuda_count, spread):
-    if spread:
-        if cuda_count < world:
-            pytest.skip(f"needs {world} GPUs")
-        return list(range(world))
-    return [0] * world
-
-
-class World:
-    def __init__(self, devices, stage_mb=8, timeout_s=10.0):
-        from torchx_b200.ddp import Communicator
-
-        self.comms = Communicator.create_local(devices, stage_mb=stage_mb)
-        self.streams = [torch.cuda.Stream(device=d) for d in devices]
-        same_device = len(set(devices)) == 1
-        for c in self.comms:
-            c.set_timeout(timeout_s)
-            if same_device:  # all kernels must be co-resident on one GPU: W ranks x grid <= #SMs (1 CTA per SM)
-                c.set_max_ctas(max(1, 128 // len(devices)))
-
-    def run(self, fn):
-        """fn(rank, comm, stream) launches that rank's work; then wait for all and check health."""
-        for r, (c, s) in enumerate(zip(self.comms, self.streams)):
-            fn(r, c, s)
-        for s in self.streams:
-            s.synchronize()
-        for c in self.comms:
-            c.check()
-
-    def close(self):
-        for c in self.comms:
-            c.close()
-
-
-def _to_dev(x, mode, device):
-    if mode == "bf16":
-        bits = oracle.f32_to_bf16_bits(x)
-        return torch.from_numpy(bits.view(np.int16).copy()).to(f"cuda:{device}").view(torch.bfloat16), bits
-    return torch.from_numpy(x.copy()).to(f"cuda:{device}"), x
-
-
-def _to_host(t, mode):
-    if mode == "bf16":
-        return t.view(torch.int16).cpu().numpy().view(np.uint16)
-    return t.cpu().numpy()
-
-
-def _check_allreduce(world_obj, n, mode, algo, kind, seed, offset=0):
+def _check_allreduce(world_obj, n, mode, algo, kind, seed, offset=0, scale=None, poke=None):
+    """One allreduce of make_inputs(kind) on every rank of `world_obj`, compared with the oracle.  Each rank's tensor lies
+    `offset` elements into its allocation, between canaries that must come through unchanged; `poke(rank, h)` may rewrite
+    rank r's elements (raw bits: fp32, or uint16 bf16 patterns) before they are uploaded."""
     W = len(world_obj.comms)
     xs = make_inputs(W, n + offset, seed, kind)
-    tens, host = [], []
+    bufs, host = [], []
     for r, c in enumerate(world_obj.comms):
-        t, h = _to_dev(xs[r], mode, c.device)
-        tens.append(t[offset:])
-        host.append(h[offset:])
-    scale = 1.0 / W
-    world_obj.run(lambda r, c, s: c.allreduce_(tens[r], scale=scale, wire=WIRE[mode], algo=algo, stream=s))
-    what = f"W={W} n={n} mode={mode} algo={algo} kind={kind}"
+        h = host_elems(xs[r][offset:], mode).copy()
+        if poke is not None:
+            poke(r, h)
+        bufs.append(Guarded(h, mode, c.device, offset=offset, seed=seed + r))
+        host.append(h)
+    if scale is None:
+        scale = 1.0 / W
+    world_obj.run(lambda r, c, s: c.allreduce_(bufs[r].t, scale=scale, wire=WIRE[mode], algo=algo, stream=s))
+    what = f"W={W} n={n} mode={mode} algo={algo} kind={kind} scale={scale!r}"
+    for r in range(W):
+        bufs[r].check(f"{what} rank={r}")
+    got = [to_host(b.t, mode) for b in bufs]
     ran_nvls = world_obj.comms[0].last_algo == "nvls"
     if ran_nvls and kind != "onehot":  # onehot: one non-zero term per element - exact on every path
         # the switch's own arithmetic (tools/nvls_probe.py, DESIGN.md 2.4): within one bf16 ulp of the exact sum
-        stats = [assert_nvls_result(_to_host(tens[r], mode), host, scale, MODES[mode], f"{what} rank={r}") for r in range(W)]
+        stats = [assert_nvls_result(got[r], host, scale, MODES[mode], f"{what} rank={r}") for r in range(W)]
         for r in range(1, W):  # every rank holds the SAME bits (one reduction per element, replicated by the switch)
-            assert_bits_equal(_to_host(tens[r], mode), _to_host(tens[0], mode), f"{what}: rank {r} vs rank 0")
+            assert_bits_equal(got[r], got[0], f"{what}: rank {r} vs rank 0")
         return stats[0]
     want = oracle.allreduce(MODES[mode], host, scale)
     for r in range(W):
-        assert_bits_equal(_to_host(tens[r], mode), want, f"{what} rank={r}")
+        assert_bits_equal(got[r], want, f"{what} rank={r}")
     return None
 
 
@@ -95,22 +56,24 @@ def test_local_pass_matches_oracle(mode):
         for kind in ("randn", "special"):
             for offset in (0, 1):
                 x = make_inputs(1, n + offset, 7, kind)[0]
-                t, h = _to_dev(x, mode, 0)
+                t, h = to_dev(x, mode, 0)
                 for scale in (1.0, 0.125, 1.0 / 3.0):
                     tt = t.clone()[offset:]
                     local_pass_(tt, scale=scale, wire=WIRE[mode])
                     torch.cuda.synchronize()
                     want = oracle.allreduce(MODES[mode], [h[offset:]], scale)
-                    assert_bits_equal(_to_host(tt, mode), want, f"local n={n} mode={mode} scale={scale} off={offset}")
+                    assert_bits_equal(to_host(tt, mode), want, f"local n={n} mode={mode} scale={scale} off={offset}")
 
 
-@pytest.mark.parametrize("world", [2, 3, 4, 8])
+@pytest.mark.parametrize("world", [2, 3, 4, 5, 6, 7, 8])
 @pytest.mark.parametrize("mode", list(MODES))
 @pytest.mark.parametrize("algo", ["oneshot", "twoshot", "twoshot_pipe", "twoshot_ll"])
 def test_allreduce_matches_oracle_one_device(world, mode, algo):
+    """SIZES 1..9 leave some ranks an empty slice; 768 * W elements end every slice (Ls = ceil(V / W) vecs) exactly on a
+    32-vec pipeline unit, one more element starts the next unit."""
     w = World([0] * world)
     try:
-        for i, n in enumerate(SIZES):
+        for i, n in enumerate(SIZES + [768 * world, 768 * world + 1]):
             _check_allreduce(w, n, mode, algo, "randn" if i % 2 == 0 else "special", seed=i)
         _check_allreduce(w, 4099, mode, algo, "randn", seed=99, offset=1)  # misaligned base pointer
         _check_allreduce(w, 1 << 12, mode, algo, "onehot", seed=0)
@@ -134,7 +97,7 @@ def test_allreduce_auto_and_chunking(world):
         w.close()
 
 
-@pytest.mark.parametrize("world", [2, 3, 4, 8])
+@pytest.mark.parametrize("world", [2, 3, 4, 5, 6, 7, 8])
 @pytest.mark.parametrize("chunk_kib", [1, 16, 4096])
 def test_pipelined_two_shot_chunking(world, chunk_kib):
     """The warp-specialised pipeline over K chunks: tiny chunks force K = 16 with ragged last cells, one huge chunk is the
@@ -148,6 +111,54 @@ def test_pipelined_two_shot_chunking(world, chunk_kib):
                 _check_allreduce(w, n, mode, "twoshot_pipe", "special" if i % 2 else "randn", seed=100 + i)
         _check_allreduce(w, 40961, "f32_wire_bf16", "twoshot_pipe", "randn", seed=7, offset=1)
         _check_allreduce(w, 1 << 14, "bf16", "twoshot_pipe", "ints", seed=8, offset=3)
+    finally:
+        w.close()
+
+
+# 1 = plain SUM (dist.all_reduce); 2^-130 turns every wire value into a bf16 / fp32 subnormal (a flush-to-zero would show);
+# 2^100 overflows the large `special` inputs to +-inf, and inf - inf makes NaN in the sum
+SCALES = [1.0, 1.0 / 3.0, 0.1, 2.0 ** -130, 2.0 ** 100]
+
+
+@pytest.mark.parametrize("world", [2, 3, 7])
+@pytest.mark.parametrize("algo", ["oneshot", "twoshot", "twoshot_pipe", "twoshot_ll"])
+def test_allreduce_any_scale_matches_oracle(world, algo):
+    w = World([0] * world)
+    try:
+        for mode in MODES:
+            for i, scale in enumerate(SCALES):
+                for n in (4099, 70001):
+                    _check_allreduce(w, n, mode, algo, "special", seed=200 + i, scale=scale)
+    finally:
+        w.close()
+
+
+def _sentinel_nans(rank, h):
+    """NaNs whose bits are the sentinel of the LL / NVLS buffers (0xFFFFFFFF: in bf16 two adjacent 0xFFFF elements, which
+    f32_to_bf16_bits would never produce) and the negative default NaN, at positions shared by all ranks and at positions
+    of this rank alone."""
+    rng = np.random.default_rng(77 + rank)
+    words = np.sort(np.concatenate([np.arange(0, h.size // 2, 97), rng.integers(0, h.size // 2, size=h.size // 64)]))
+    if h.dtype == np.uint16:
+        h[2 * words] = 0xFFFF
+        h[2 * words + 1] = 0xFFFF
+        h[2 * words[::3] + 1] = 0xFFC0  # every third pair: a negative NaN in the upper half of the word
+    else:
+        bits = h.view(np.uint32)
+        bits[2 * words] = 0xFFFFFFFF
+        bits[2 * words + 1] = 0xFFC00000
+
+
+@pytest.mark.parametrize("world", [2, 3, 7])
+def test_sentinel_bit_patterns_in_the_input(world):
+    """Input words equal to the LL sentinel must come out as NaN and must not be taken for "not written yet" (which
+    would end in a peer-wait timeout that check() reports)."""
+    w = World([0] * world)
+    try:
+        for mode in MODES:
+            for n in (4099, 70001, (1 << 18) + 5):
+                _check_allreduce(w, n, mode, "twoshot_ll", "randn", seed=n, poke=_sentinel_nans)
+                _check_allreduce(w, n, mode, "twoshot_ll", "randn", seed=n, scale=1.0, poke=_sentinel_nans)
     finally:
         w.close()
 
@@ -240,7 +251,7 @@ def test_dead_peer_times_out_instead_of_hanging():
 def test_allreduce_across_devices(world, algo, cuda_count):
     """Real NVLink/NVSwitch peers (skipped on a 1-GPU box).  In-process worlds over distinct devices use the VMM arena and,
     where the fabric offers it, the multicast object - the same mappings as the one-process-per-GPU path minus fd passing."""
-    devs = _devices(world, cuda_count, spread=True)
+    devs = devices(world, cuda_count, spread=True)
     w = World(devs, stage_mb=64)
     try:
         if algo == "nvls" and not w.comms[0].has_multicast:
@@ -261,10 +272,25 @@ def test_allreduce_across_devices(world, algo, cuda_count):
 
 
 @pytest.mark.parametrize("world", [2, 4, 8])
+@pytest.mark.parametrize("algo", ["twoshot_ll", "nvls"])
+def test_sentinel_bit_patterns_across_devices(world, algo, cuda_count):
+    """The NVLS output buffers use the same sentinel as LL: an input word equal to it must not stall the switch path."""
+    w = World(devices(world, cuda_count, spread=True), stage_mb=64)
+    try:
+        if algo == "nvls" and not w.comms[0].has_multicast:
+            pytest.skip("no NVSwitch multicast on this box")
+        for mode in ("f32_wire_bf16", "bf16") if algo == "nvls" else MODES:
+            for n in (4099, (1 << 20) + 5):
+                _check_allreduce(w, n, mode, algo, "randn", seed=n, poke=_sentinel_nans)
+    finally:
+        w.close()
+
+
+@pytest.mark.parametrize("world", [2, 4, 8])
 def test_messages_larger_than_a_stage_across_devices(world, cuda_count):
     """stage_mb=1: every algorithm has to cut the message into several launches that alternate between the two staging
     buffers while the peers run skewed on real NVLink."""
-    devs = _devices(world, cuda_count, spread=True)
+    devs = devices(world, cuda_count, spread=True)
     w = World(devs, stage_mb=1)
     try:
         for c in w.comms:

@@ -1069,15 +1069,18 @@ int b2_allreduce(b2_comm_t* c, void* buf, size_t n_elems, int mode, float scale,
 int b2_allreduce_gather(b2_comm_t* c, void* out, size_t n_elems, const b2_segment_t* segments, int n_segments, int mode,
                         float scale, int algo, void* stream) {
   if (n_elems == 0) return B2_OK;
-  if (!segments || n_segments <= 0 || n_segments > B2_MAX_SEGMENTS)
+  if (!segments) return fail(B2_EINVAL, "b2_allreduce_gather: null segment table");
+  if (n_segments <= 0 || n_segments > B2_MAX_SEGMENTS)
     return fail(B2_EINVAL, "b2_allreduce_gather: need 1..%d segments (got %d)", B2_MAX_SEGMENTS, n_segments);
   Src src;
   src.nseg = n_segments;
   src.off = 0;
   unsigned long long at = 0;
   for (int i = 0; i < n_segments; ++i) {
-    if (segments[i].begin != at || segments[i].end <= at || !segments[i].src)
+    if (segments[i].begin != at)
       return fail(B2_EINVAL, "b2_allreduce_gather: segment %d does not continue the bucket at element %llu", i, at);
+    if (segments[i].end <= at) return fail(B2_EINVAL, "b2_allreduce_gather: segment %d is empty", i);
+    if (!segments[i].src) return fail(B2_EINVAL, "b2_allreduce_gather: segment %d has a null src", i);
     src.ptr[i] = segments[i].src;
     src.begin[i] = at;
     at = segments[i].end;
